@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — formula-images/sec of one full im2latex train step (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32] [--dump-outputs DIR]
 
 N=1 workload = BASELINE.json configs[1]: batch 64, 1x128x512 images, 6-conv encoder + 512-d attention LSTM
 decoder, vocab 500, every caption padded to T=150 decode steps (the reference trains on PADs,
@@ -9,10 +9,18 @@ img2seq_torch.py:144), bf16 storage / fp32 accumulate.  N>1 (torchrun, one rank 
 batch on every rank (weak scaling), NCCL all-reduce of the two gradient buckets.
 
 A "step" = encoder fwd -> decoder fwd -> loss -> decoder bwd -> encoder bwd -> [all-reduce] -> Adam, nothing
-skipped.  `value` times K steps with inputs resident in HBM (CUDA events, max over ranks); `e2e` times the same
-K steps through Img2SeqModel.train_step with PINNED HOST inputs (H2D inside) and a D2H read of the loss.
+skipped.  `value` times K steps with inputs resident in HBM (CUDA events around each step, summed; max over ranks);
+`e2e` times K steps through Img2SeqModel.train_step with PINNED HOST inputs (H2D inside) and a D2H read of the loss.
 `--impl reference` times the reference's CPU algorithm (oracle port, un-hoisted exactly as the reference
 executes it) on the host cores of rank 0.
+
+The batch, the initial weights and the dropout seed are seeded, and every warm-up and timed step of `value` trains
+the same state (the initial weights, zero Adam moments; restored between steps, outside the timed intervals): the
+backward adds partial sums with fp32 atomics in varying order, and carried from step to step those last-bit
+differences grow through the recurrence, the ReLU / max-pool tie-breaks and Adam until two runs train different
+models.  So a step's inputs are the same on every run, and so is its loss, which the forward computes without atomics.
+`--dump-outputs DIR` writes what the last timed step returned to its caller (Img2SeqModel.train_step) as
+DIR/loss.npy: [total, ce, reg, n_valid], float32.  Two builds run with the same arguments can then be compared.
 """
 import argparse
 import json
@@ -119,6 +127,14 @@ def log(*a):
     print("[bench %.1fs]" % (time.time() - T0), *a, file=sys.stderr, flush=True)
 
 
+def dump_outputs(out_dir, loss):
+    """The loss vector train_step returned, as DIR/loss.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    log("wrote %s" % os.path.join(out_dir, "loss.npy"))
+
+
 T0 = time.time()
 
 
@@ -135,11 +151,14 @@ def main():
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-decode", action="store_true", help="omit the cfg #5 decode probe (N=1 only)")
     ap.add_argument("--workload", default="cfg2", choices=["cfg2", "cfg4"], help="cfg4 = the row-encoder / two-layer EXTENSION")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss vector of the last timed step as DIR/loss.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs dumps the GPU train step; --impl reference does not run it")
         return run_reference(args, rank)
 
     import torch
@@ -172,6 +191,7 @@ def main():
         from latex_ocr_b200.ext import Img2SeqRowModel as ModelCls
     else:
         ModelCls = Img2SeqModel
+    torch.manual_seed(1234 + rank)             # initial weights and the decoder's dropout seed
     model = ModelCls(Cfg(), vocab=SimpleVocab(c["V"]), device="cuda:%d" % local, precision=args.precision, impl=kernels)
     model.build_train()
     model.train_mode(True)                     # dropout active, like the reference's training loop
@@ -187,9 +207,20 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    # the state every step of the device-resident timing trains (see the module docstring)
+    stores = model._stores()
+    initial = [{k: getattr(S, k).clone() for k in ("master", "m", "v", "adam_state", "shadow") if getattr(S, k) is not None}
+               for S in stores]
+
+    def restore_initial_state():
+        for S, snap in zip(stores, initial):
+            for k, v in snap.items():
+                getattr(S, k).copy_(v)
+
     log("model built; warm-up")
     # ---- device-resident timing ---------------------------------------------------------------------
     for _ in range(args.warmup):
+        restore_initial_state()
         model.train_step(img_dev, formula_dev)
     barrier()
     log("warm-up done; timing")
@@ -197,19 +228,23 @@ def main():
     if rank == 0:
         sampler.start()
     l0 = _lib.launch_count()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     barrier()
-    e0.record()
-    for _ in range(args.steps):
+    for a, b in ev:
+        restore_initial_state()
+        a.record()
         loss = model.train_step(img_dev, formula_dev)
-    e1.record()
+        b.record()
     barrier()
-    ms = e0.elapsed_time(e1) / args.steps
+    ms = sum(a.elapsed_time(b) for a, b in ev) / args.steps
     clocks = sampler.stop() if rank == 0 else None
     launches_eager = _lib.launch_count() - l0
     final_loss = float(loss[0].item())
     log("device-resident: %.2f ms/step" % ms)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss)
     # ---- end-to-end timing (pinned host inputs, H2D + loss D2H every step) -----------------------------
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     for _ in range(2):
         model.getLoss(img_pin, formula_pin)
     barrier()

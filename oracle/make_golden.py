@@ -5,7 +5,8 @@ Weights are NOT stored (9.5 M floats): every case records the ``init_params`` se
 reference modules are loaded with exactly those tensors through ``load_state_dict``.  Stored:
 inputs' seeds/shapes, loss, scores, alphas, encoder output, bias gradients in full, and for
 the big weight gradients their sum / abs-sum / first 256 values — plus a 3-step Adam loss
-trajectory.  The GPU box has no /root/reference: tests read only these files.
+trajectory.  Outputs of more than OUTPUT_FULL_MAX elements are stored as the same summaries, so
+that every file stays under 1 MB.  Tests read only these files, never the reference itself.
 """
 import os
 import sys
@@ -24,11 +25,12 @@ CASES = {
     "tiny_nopos": dict(B=2, H=48, W=64, V=37, tmin=2, tmax=5, train=False, positional=False, pseed=13, dseed=23),
     "cfg1": dict(B=4, H=64, W=256, V=100, tmin=8, tmax=32, train=False, positional=True, pseed=14, dseed=24),
     # BASELINE.json configs[1] shapes (R = 14*62 = 868, T = 150, V = 500) on a B=8 sample of the batch, dropout active:
-    # the exact tiles / 150-step recurrence the bench runs.  Summaries only (strided samples), ~1.5 MB.
+    # the exact tiles / 150-step recurrence the bench runs.  Summaries only (strided samples), ~0.6 MB.
     "cfg2": dict(B=8, H=128, W=512, V=500, tmin=150, tmax=150, train=True, positional=True, pseed=16, dseed=26, summaries_only=True),
 }
 
 SAMPLE_N = 8192
+OUTPUT_FULL_MAX = 65536
 
 
 def summarize(g):
@@ -85,13 +87,9 @@ def run_case(name, c):
         loss.backward()
         if step == 0:
             rec["loss"] = loss.item()
-            if c.get("summaries_only"):
-                big = summarize({"scores": scores, "alphas": alphas, "enc_out": enc(img)})
-                rec["scores"], rec["alphas"], rec["enc_out"] = big["scores"], big["alphas"], big["enc_out"]
-            else:
-                rec["scores"] = scores.detach().clone()
-                rec["alphas"] = alphas.detach().clone()
-                rec["enc_out"] = enc(img).detach().clone()
+            for k, v in (("scores", scores), ("alphas", alphas), ("enc_out", enc(img))):
+                big = c.get("summaries_only") or v.numel() > OUTPUT_FULL_MAX
+                rec[k] = summarize({k: v})[k] if big else v.detach().clone()
             rec["grad_enc"] = summarize({k: v.grad for k, v in enc.named_parameters()})
             rec["grad_dec"] = summarize({k: v.grad for k, v in dec.named_parameters()})
         od.step()
@@ -99,13 +97,11 @@ def run_case(name, c):
         traj.append(-loss.item())                              # getLoss returns -loss (:172)
     rec["get_loss_trajectory"] = traj
     rec["mask_seed"] = mask_seed
-    rec["params_after_3_steps"] = summarize({**{"enc." + k: v for k, v in enc.state_dict().items()},
-                                             **{"dec." + k: v for k, v in dec.state_dict().items()}})
     # self-check: restatement reproduces it bit for bit right now
     mask = dropout_masks(mask_seed, c["B"], T, 512) if c["train"] else None
     l2, aux = rm.get_loss(pe, pd, img, formula, dropout_mask=mask, positional=c["positional"])
     assert abs(l2.item() - rec["loss"]) == 0.0, (name, l2.item(), rec["loss"])
-    if c.get("summaries_only"):
+    if isinstance(rec["scores"], dict):
         assert (strided_sample(aux["scores"])["sample"] - rec["scores"]["sample"]).abs().max().item() == 0.0
     else:
         assert (aux["scores"] - rec["scores"]).abs().max().item() == 0.0
@@ -131,6 +127,24 @@ def run_cnn_variant():
     print("cnn_variant", tuple(out.shape), "bytes", os.path.getsize(os.path.join(OUT, "cnn_variant.pt")))
 
 
+def run_reference_outputs():
+    """The reference's own forward outputs, in full: getLoss (loss, scores, alphas) in eval mode, and
+    DecoderWithAttention.forward with ragged caption lengths (the shrinking batch, seq2seq_torch.py:308)."""
+    c = dict(B=2, H=32, W=96, V=50, tmin=3, tmax=6, pseed=21, dseed=22, lengths=[[7], [4]])
+    pe, pd = rm.init_params(c["V"], seed=c["pseed"])
+    enc, dec = ref_shim.build_reference_models(c["V"])
+    enc.load_state_dict(pe)
+    dec.load_state_dict(pd)
+    dec.eval()
+    img, formula = rm.synthetic_batch(c["B"], c["H"], c["W"], c["V"], c["tmin"], c["tmax"], seed=c["dseed"])
+    loss, scores, alphas = ref_shim.ref_get_loss(enc, dec, img, formula)
+    r_scores, _, r_lengths, r_alphas, _ = dec(enc(img), formula, torch.tensor(c["lengths"]))
+    rec = dict(case=c, torch=torch.__version__, loss=loss.item(), scores=scores.detach().clone(), alphas=alphas.detach().clone(),
+               ragged_scores=r_scores.detach().clone(), ragged_alphas=r_alphas.detach().clone(), ragged_decode_lengths=list(r_lengths))
+    torch.save(rec, os.path.join(OUT, "reference_outputs.pt"))
+    print("reference_outputs loss", rec["loss"], "bytes", os.path.getsize(os.path.join(OUT, "reference_outputs.pt")))
+
+
 def main():
     if not ref_shim.reference_available():
         sys.exit("reference tree not available; golden files can only be regenerated in the build container")
@@ -143,6 +157,8 @@ def main():
         run_case(name, c)
     if not only or "cnn_variant" in only:
         run_cnn_variant()
+    if not only or "reference_outputs" in only:
+        run_reference_outputs()
 
 
 if __name__ == "__main__":

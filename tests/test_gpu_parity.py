@@ -54,8 +54,16 @@ def test_encoder_forward_vs_golden(name):
     c, pe, pd, img, formula = _case_inputs(rec)
     m = build_model(c["V"], pe, pd, "fp32", positional=c["positional"])
     out = m.encoder(img.cuda())
-    assert out.shape == rec["enc_out"].shape
-    assert relerr(out, rec["enc_out"]) < 1e-4
+    want = rec["enc_out"]
+    if isinstance(want, dict):
+        # cfg1 stores a strided sample of the reference output; every element is compared with the CPU oracle, the
+        # restatement that tests/test_oracle_pinned.py pins to the reference
+        assert tuple(out.shape) == want["shape"]
+        s = _sample_of(out, want)
+        assert (s - want["sample"].double()).abs().max().item() < 1e-4 * want["sample"].abs().max().item()
+        want = _oracle().encoder_forward(pe, img, positional=c["positional"])
+    assert out.shape == want.shape
+    assert relerr(out, want) < 1e-4
 
 
 @pytest.mark.parametrize("name", ["tiny_eval", "tiny_nopos", "tiny_train", "cfg1"])

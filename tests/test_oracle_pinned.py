@@ -1,11 +1,10 @@
 """CPU (-m "not gpu"): the oracle restatement against the golden fixtures generated from the UNMODIFIED
-reference (oracle/make_golden.py), and — when /root/reference is present — against the live reference."""
+reference (oracle/make_golden.py)."""
 import pytest
 import torch
 
 from util import load_golden, relerr
 from oracle import ref_model as rm
-from oracle import ref_shim
 
 
 def _inputs(rec):
@@ -78,24 +77,23 @@ def test_manual_backward_equals_autograd():
     assert (enc.grad - denc).abs().max().item() < 1e-14
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference tree only exists in the build container")
-def test_restatement_matches_live_reference():
-    V = 50
-    pe, pd = rm.init_params(V, seed=21)
-    enc, dec = ref_shim.build_reference_models(V)
-    enc.load_state_dict(pe)
-    dec.load_state_dict(pd)
-    dec.eval()
-    img, formula = rm.synthetic_batch(2, 32, 96, V, 3, 6, seed=22)
-    loss_ref, s_ref, a_ref = ref_shim.ref_get_loss(enc, dec, img, formula)
+def test_restatement_matches_reference_outputs():
+    """The reference's forward outputs stored in full (oracle/make_golden.py, where the restatement reproduced them bit for
+    bit).  A CPU with another thread count or vector width may sum in another order, so floats are held to 1e-6."""
+    torch.set_num_threads(8)
+    rec = load_golden("reference_outputs")
+    c = rec["case"]
+    pe, pd = rm.init_params(c["V"], seed=c["pseed"])
+    img, formula = rm.synthetic_batch(c["B"], c["H"], c["W"], c["V"], c["tmin"], c["tmax"], seed=c["dseed"])
     loss, aux = rm.get_loss(pe, pd, img, formula)
-    assert loss.item() == loss_ref.item()
-    assert torch.equal(aux["scores"], s_ref) and torch.equal(aux["alphas"], a_ref)
+    assert abs(loss.item() - rec["loss"]) <= 1e-6 * abs(rec["loss"])
+    assert aux["scores"].shape == rec["scores"].shape and relerr(aux["scores"], rec["scores"]) < 1e-6
+    assert aux["alphas"].shape == rec["alphas"].shape and relerr(aux["alphas"], rec["alphas"]) < 1e-6
     # ragged lengths (shrinking batch) through DecoderWithAttention.forward
-    lengths = torch.tensor([[7], [4]])
-    out_ref = dec(enc(img), formula, lengths)
-    out = rm.decoder_forward(pd, rm.encoder_forward(pe, img), formula, lengths)
-    assert torch.equal(out[0], out_ref[0]) and torch.equal(out[3], out_ref[3]) and out[2] == out_ref[2]
+    out = rm.decoder_forward(pd, rm.encoder_forward(pe, img), formula, torch.tensor(c["lengths"]))
+    assert out[2] == rec["ragged_decode_lengths"]
+    assert out[0].shape == rec["ragged_scores"].shape and relerr(out[0], rec["ragged_scores"]) < 1e-6
+    assert out[3].shape == rec["ragged_alphas"].shape and relerr(out[3], rec["ragged_alphas"]) < 1e-6
 
 
 def test_tf_flavour_oracle_self_consistency():
