@@ -173,6 +173,7 @@ int lo_attention_forward_mask(const void* att1, const void* enc, int dt, const f
  * att2 / gate [B][o1_stride] fp32 as the forward left them (gate after the sigmoid; NULL = ungated context) ; alpha / de
  * [B][alpha_stride] ; ctx / dctx_out [B][C] ; dgctx [B][dg_stride] ; dreg [B][dreg_stride] and sreg [B][sreg_stride] may be NULL ;
  * datt2 / dgp [B][dcat_stride] ; dwf_part (optional) [B][A] += sum_r de_r relu(att1_r + att2) (full_att.weight gradient).
+ * dgp and dctx_out may be NULL; with gate NULL, dctx = dgctx and dgp (when given) is written with zeros.
  * d att1 and d enc are NOT produced here: they are hoisted out of the time loop (see lo_decoder_backward).
  * relu_mask (optional): the bits lo_attention_forward_mask stored; att1 is then NOT read, and dwf_part (optional) receives only the
  * att2 term of the full_att.weight gradient, sum_r de_r [on] att2_a — the term that needs att1 itself, sum_r de_r [on] att1_ra, is

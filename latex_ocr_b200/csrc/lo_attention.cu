@@ -168,6 +168,12 @@ __global__ void __launch_bounds__(AP_THREADS, LO_ATT_MINB) attention_fwd_pipe_ke
     pdl_trigger();
 #pragma unroll
     for (int j = 0; j < NVA; j++) ld8(att2 + (int64_t)b * att2_stride + (j * 32 + lane) * 8, a2 + j * 8);
+    // mask bits: the score loop works on n = (0 - att2) - att1 = -(att1 + att2), whose SIGN bit is set exactly when att1 + att2 > 0.
+    // The negation rounds symmetrically, an exact cancellation gives +0, and 0 - att2 is never -0, so no pair of zeros gives -0 either.
+    if constexpr (MK) {
+#pragma unroll
+      for (int i = 0; i < NVA * 8; i++) a2[i] = 0.f - a2[i];
+    }
     // cluster mode: the gate pre-activation of the channel this thread finalises after the combine (one L2 round trip off the tail)
     if (CL && gate_pre && (int)threadIdx.x < (CHC + nsplit - 1) / nsplit && sp * ((CHC + nsplit - 1) / nsplit) + (int)threadIdx.x < CHC)
       gate_pf = gate_pre[(int64_t)b * gate_stride + sp * ((CHC + nsplit - 1) / nsplit) + threadIdx.x];
@@ -199,23 +205,34 @@ __global__ void __launch_bounds__(AP_THREADS, LO_ATT_MINB) attention_fwd_pipe_ke
           uint32_t bits = 0;
 #pragma unroll
           for (int q = 0; q < 8; q++) {
-            const float pre = v[q] + a2[j * 8 + q];
-            // one funnel shift per element collects the SIGN bits (element q -> bit 7-q); pre > 0 <=> sign clear, except for
-            // pre == +0 exactly, where the ReLU subgradient is a convention and which a sum of a bf16 and an fp32 never hits
-            if (MK) bits = __funnelshift_l(__float_as_uint(pre), bits, 1);
+            // one funnel shift per element collects the sign bits of n = -pre (element q -> bit 7-q): bit = pre > 0, +0 included
+            float pre;
+            if constexpr (MK) {
+              const float n = a2[j * 8 + q] - v[q];
+              bits = __funnelshift_l(__float_as_uint(n), bits, 1);
+              pre = -n;
+            } else {
+              pre = v[q] + a2[j * 8 + q];
+            }
             e0 = fmaf(wv[j * 8 + q], att_act<ACT, sizeof(T) == 2>(pre), e0);
           }
-          if (MK) mrow[(int64_t)((row + ra) >> 1) * (CHA / 4) + (j * 32 + lane) * 2 + ((row + ra) & 1)] = (uint8_t)(~bits);
+          if (MK) mrow[(int64_t)((row + ra) >> 1) * (CHA / 4) + (j * 32 + lane) * 2 + ((row + ra) & 1)] = (uint8_t)bits;
           if (two) {
             lds8(sa + ((uint32_t)rb * CHA + (j * 32 + lane) * 8) * ES, v, (const T*)nullptr);
             bits = 0;
 #pragma unroll
             for (int q = 0; q < 8; q++) {
-              const float pre = v[q] + a2[j * 8 + q];
-              if (MK) bits = __funnelshift_l(__float_as_uint(pre), bits, 1);
+              float pre;
+              if constexpr (MK) {
+                const float n = a2[j * 8 + q] - v[q];
+                bits = __funnelshift_l(__float_as_uint(n), bits, 1);
+                pre = -n;
+              } else {
+                pre = v[q] + a2[j * 8 + q];
+              }
               e1 = fmaf(wv[j * 8 + q], att_act<ACT, sizeof(T) == 2>(pre), e1);
             }
-            if (MK) mrow[(int64_t)((row + rb) >> 1) * (CHA / 4) + (j * 32 + lane) * 2 + ((row + rb) & 1)] = (uint8_t)(~bits);
+            if (MK) mrow[(int64_t)((row + rb) >> 1) * (CHA / 4) + (j * 32 + lane) * 2 + ((row + rb) & 1)] = (uint8_t)bits;
           }
         }
         e0 = warp_sum(e0);
@@ -1412,6 +1429,7 @@ extern "C" int lo_get_option(const char* name) {
   if (!strcmp(name, "dbg_skip")) return lo::g_opt_dbg_skip;
   if (!strcmp(name, "conv_mc")) return lo::g_opt_conv_mc;
   if (!strcmp(name, "att_cluster")) return lo::g_opt_att_cluster;
+  if (!strcmp(name, "att_nsplit")) return lo::g_opt_att_nsplit;
   if (!strcmp(name, "pdl")) return lo::g_opt_pdl;
   if (!strcmp(name, "conv_persist")) return lo::g_opt_conv_persist;
   if (!strcmp(name, "wgrad256")) return lo::g_opt_wgrad256;

@@ -218,7 +218,8 @@ struct AttBwdArgs {
   int act;
   int a_ch;
   const uint8_t* mask_in;   // optional (ReLU score only): the forward's mask bits; the kernel then streams enc + 1 bit per att1
-                            // element instead of enc + att1 (d w_full must then come from the post-loop sweep: dwf_part unused)
+                            // element instead of enc + att1 (dwf_part then receives only the att2 term of d w_full; the att1 term
+                            // comes from the post-loop sweep)
   int abi = 0;         // as in AttFwdArgs
 };
 extern int g_opt_att_pipe;
