@@ -407,6 +407,28 @@ int64_t lo_lstm_seq_workspace_bytes(const lo_lstm_seq_args* a);
 int lo_lstm_seq_forward(const lo_lstm_seq_args* a, void* stream);
 int lo_lstm_seq_backward(const lo_lstm_seq_args* a, void* stream);
 
+/* EXTENSION: greedy / beam decoding of the two-layer decoder (layer 1 = the attention LSTM of lo_decoder_args, layer 2 =
+ * nn.LSTMCell(D, D) over h1_t with zero initial state, logits_t = fc(h2_t); no dropout at decode time).  Layer 2 runs inside the
+ * time loop, one step per step: gates2 = h1_t W_ih^T + h2_{t-1} W_hh^T + b_ih + b_hh, then the cell (gate order i,f,g,o).
+ * In beam search its state (h2, c2) is gathered by parents like layer 1's.  Loop rules, outputs and limits are those of
+ * lo_decoder_greedy_hist / lo_decoder_beam_div. */
+typedef struct lo_dec2_args {
+  int32_t D;               /* hidden width; must equal lo_decoder_args.D */
+  int32_t dt;              /* storage of the weight shadows: LO_F32 | LO_BF16 */
+  int32_t impl;            /* LO_IMPL_SIMT | LO_IMPL_TC (tensor-core GEMMs; used when the decoder runs its bf16 mirrors) */
+  const void* w_ih;        /* dt [4D][D] */
+  const void* w_hh;        /* dt [4D][D] */
+  const float* b_ih; const float* b_hh;   /* fp32 [4D] */
+  void* ws;                /* lo_dec2_workspace_bytes(B, D) bytes, B = lo_decoder_args.B; no initialisation needed */
+} lo_dec2_args;
+int64_t lo_sizeof_dec2_args(void);
+int64_t lo_dec2_workspace_bytes(int B, int D);
+int lo_decoder2_greedy_hist(const lo_decoder_args* a, const lo_dec2_args* l2, int64_t start_id, int64_t end_id, int max_steps,
+                            int64_t* tokens, int32_t* finished, int32_t* fin_hist, void* stream);
+int lo_decoder2_beam_div(const lo_decoder_args* a, const lo_dec2_args* l2, int64_t start_id, int64_t end_id, int max_steps,
+                         int64_t* ids, int64_t* parents, int32_t* fin_hist, float* logp, float div_gamma, float div_prob,
+                         const float* div_u, const uint64_t* div_state, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Optimiser: torch.optim.Adam defaults (img2seq_torch.py:86-87, :168-170) on one flat buffer.
  * state_dev: float[2] = {step (as float), lr}; step is incremented on the device so the call is

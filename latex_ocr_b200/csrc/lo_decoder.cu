@@ -1142,6 +1142,9 @@ static inline Rows chain_rows(const lo_decoder_args* a, const Dims& d, int chain
 
 }  // namespace lo
 
+// greedy / beam decode loops (one- and two-layer decoder) and the two-layer decode entry points
+#include "lo_decoder2.cuh"
+
 using namespace lo;
 
 extern "C" {
@@ -1691,33 +1694,7 @@ int lo_decoder_backward(const lo_decoder_args* a, void* stream) {
 
 int lo_decoder_greedy_hist(const lo_decoder_args* a, int64_t start_id, int64_t end_id, int max_steps, int64_t* tokens,
                            int32_t* finished, int32_t* fin_hist, void* stream) {
-  LO_TRY(check_args(a));
-  LO_CHECK_ARG(tokens && finished && max_steps > 0 && max_steps <= a->T, "tokens/finished/max_steps (<= T capacity)");
-  cudaStream_t st = (cudaStream_t)stream;
-  const Dims d = dims(a);
-  int64_t* next_tok = (int64_t*)a->sreg;          // scratch: [B] int64 fits in sreg [B][>=2] floats
-  fill_i64_kernel<<<cdiv(d.B, 128), 128, 0, st>>>(next_tok, start_id, d.B);
-  LO_LAUNCH_OK();
-  LO_CUDA(cudaMemsetAsync(finished, 0, (size_t)d.B * 4, st));
-  LO_TRY(forward_prologue(a, d, st));
-  const BfViews bvg = bf_views(a, d);
-  for (int t = 0; t < max_steps; t++) {
-    LO_TRY(forward_step(a, d, t, Rows{0, d.B, a->work, 0}, next_tok, 1, nullptr, 0, nullptr, st));
-    // logits_t = fc(h_t)   (no dropout at decode time)
-    if (bvg.on)      // bf16 mirror of h_t: mma.sync kernel for <= 64 rows (the dispatcher falls back to CUDA cores otherwise)
-      LO_TRY(gemm_nt(bvg.hall + (int64_t)(t + 1) * d.B * d.D, LO_BF16, d.D, a->w_fc, LO_BF16, d.D, a->logits, LO_F32, d.V, d.B, d.V, d.D,
-                     a->b_fc, 0, 0, LO_IMPL_TC, st));
-    else
-      LO_TRY(gemm_nt(a->hall + (int64_t)(t + 1) * d.B * d.D, LO_F32, d.D, a->w_fc, a->dt, d.D, a->logits, LO_F32, d.V, d.B, d.V, d.D,
-                     a->b_fc, 0, 0, LO_IMPL_SIMT, st));
-    argmax_kernel<<<cdiv(d.B, 8), 256, 0, st>>>(a->logits, d.V, tokens + t, max_steps, next_tok, finished, end_id, d.B);
-    LO_LAUNCH_OK();
-    if (fin_hist) {
-      fin_hist_kernel<<<cdiv(d.B, 128), 128, 0, st>>>(finished, fin_hist + t, max_steps, d.B);
-      LO_LAUNCH_OK();
-    }
-  }
-  return LO_OK;
+  return greedy_loop(a, nullptr, start_id, end_id, max_steps, tokens, finished, fin_hist, (cudaStream_t)stream);
 }
 
 int lo_decoder_greedy(const lo_decoder_args* a, int64_t start_id, int64_t end_id, int max_steps, int64_t* tokens,
@@ -1733,57 +1710,8 @@ int lo_decoder_beam(const lo_decoder_args* a, int64_t start_id, int64_t end_id, 
 int lo_decoder_beam_div(const lo_decoder_args* a, int64_t start_id, int64_t end_id, int max_steps, int64_t* ids, int64_t* parents,
                         int32_t* fin_hist, float* logp, float div_gamma, float div_prob, const float* div_u,
                         const uint64_t* div_state, void* stream) {
-  LO_TRY(check_args(a));
-  const bool div_on = !(div_gamma == 1.f || div_prob == 0.f);               // beam_search_decoder_cell.py:270-273
-  LO_CHECK_ARG(!div_on || (div_gamma > 0.f && (div_u || div_state)), "diversity penalty needs gamma > 0 and div_u or div_state");
-  const int beam = a->rows_per_img;
-  LO_CHECK_ARG(beam >= 1 && beam <= LO_BEAM_MAX && a->B % beam == 0, "1 <= beam (rows_per_img) <= 16, B % beam == 0");
-  LO_CHECK_ARG(ids && parents && fin_hist && logp && max_steps > 0 && max_steps <= a->T, "outputs / max_steps (<= T capacity)");
-  LO_CHECK_ARG((size_t)beam * a->V * 4 * (div_on ? 2 : 1) <= 200 * 1024, "beam*V too large for the shared-memory top-k");
-  cudaStream_t st = (cudaStream_t)stream;
-  const Dims d = dims(a);
-  const int n_img = d.B / beam;
-  // scratch: next tokens (int64 [B]) in sreg, finished + parent rows (int32 [B] each) in row_loss
-  int64_t* next_tok = (int64_t*)a->sreg;
-  int32_t* finished = (int32_t*)a->row_loss;
-  int32_t* parent_rows = finished + d.B;
-  LO_CHECK_ARG((int64_t)d.B * d.T >= 2 * d.B, "row_loss scratch too small");
-  fill_i64_kernel<<<cdiv(d.B, 128), 128, 0, st>>>(next_tok, start_id, d.B);
-  LO_LAUNCH_OK();
-  LO_CUDA(cudaMemsetAsync(finished, 0, (size_t)d.B * 4, st));
-  LO_CUDA(cudaMemsetAsync(logp, 0, (size_t)d.B * 4, st));          // initial log-probs are zeros (:106-107)
-  LO_TRY(forward_prologue(a, d, st));
-  const BfViews bv = bf_views(a, d);
-  const size_t smem = (size_t)beam * d.V * 4 * (div_on ? 2 : 1);
-  static bool attr = false;
-  if (!attr && smem > 48 * 1024) {
-    LO_CUDA(cudaFuncSetAttribute(beam_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    attr = true;
-  }
-  for (int t = 0; t < max_steps; t++) {
-    LO_TRY(forward_step(a, d, t, Rows{0, d.B, a->work, 0}, next_tok, 1, nullptr, 0, nullptr, st));
-    float* h_new = a->hall + (int64_t)(t + 1) * d.B * d.D;
-    float* c_new = a->call + (int64_t)(t + 1) * d.B * d.D;
-    if (bv.on)       // bf16 mirror of h_t -> mma.sync kernel (row blocks of 64), CUDA cores otherwise
-      LO_TRY(gemm_nt(bv.hall + (int64_t)(t + 1) * d.B * d.D, LO_BF16, d.D, a->w_fc, LO_BF16, d.D, a->logits, LO_F32, d.V, d.B, d.V, d.D,
-                     a->b_fc, 0, 0, LO_IMPL_TC, st));
-    else
-      LO_TRY(gemm_nt(h_new, LO_F32, d.D, a->w_fc, a->dt, d.D, a->logits, LO_F32, d.V, d.B, d.V, d.D, a->b_fc, 0, 0, LO_IMPL_SIMT, st));
-    beam_step_kernel<<<n_img, 256, smem, st>>>(a->logits, d.V, beam, t, end_id, logp, finished, ids, parents, fin_hist, next_tok,
-                                               parent_rows, max_steps, div_on ? logf(div_gamma) : 0.f, div_on ? div_prob : 0.f,
-                                               div_u ? div_u + (int64_t)t * d.B * d.V : (const float*)nullptr,
-                                               (const unsigned long long*)div_state);
-    LO_LAUNCH_OK();
-    // reorder the recurrent state by parents (through gtmp as a temporary)
-    gather_rows_kernel<<<cdiv((long)d.B * d.D, 256), 256, 0, st>>>(h_new, parent_rows, a->gtmp, d.B, d.D);
-    LO_LAUNCH_OK();
-    gather_rows_kernel<<<cdiv((long)d.B * d.D, 256), 256, 0, st>>>(c_new, parent_rows, a->gtmp + (int64_t)d.B * d.D, d.B, d.D);
-    LO_LAUNCH_OK();
-    LO_CUDA(cudaMemcpyAsync(h_new, a->gtmp, (size_t)d.B * d.D * 4, cudaMemcpyDeviceToDevice, st));
-    LO_CUDA(cudaMemcpyAsync(c_new, a->gtmp + (int64_t)d.B * d.D, (size_t)d.B * d.D * 4, cudaMemcpyDeviceToDevice, st));
-    if (bv.on) LO_TRY(lo_cast(h_new, LO_F32, bv.hall + (int64_t)(t + 1) * d.B * d.D, LO_BF16, (int64_t)d.B * d.D, stream));
-  }
-  return LO_OK;
+  return beam_loop(a, nullptr, start_id, end_id, max_steps, ids, parents, fin_hist, logp, div_gamma, div_prob, div_u, div_state,
+                   (cudaStream_t)stream);
 }
 
 }  // extern "C"

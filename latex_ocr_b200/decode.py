@@ -28,6 +28,11 @@ def _n_steps(fin_hist):
 
 def _prepare(model, img, rows_per_img, max_steps):
     enc = model.encoder.forward_raw(img.to(model.device).float(), need_grad=False)
+    return _prepare_enc(model, enc, rows_per_img, max_steps)
+
+
+def _prepare_enc(model, enc, rows_per_img, max_steps):
+    """enc: the storage-dtype encoder output [N,H',W',C] (CUDA) -> (decoder argument block, workspace, N)."""
     N = enc.shape[0]
     R = enc.shape[1] * enc.shape[2]
     enc_flat = enc.view(N, R, enc.shape[3])
@@ -47,15 +52,22 @@ def greedy_decode(model, img, start_id, end_id, max_length_formula=150, return_a
     returns the attention weights of every step, [N, steps, R] fp32 on the CPU — what the reference collects in
     ``attention_mechanism.ctx_vector`` for visualize_attention.py (attention_mechanism.py:96-121)."""
     L = _lib.lib()
+    return _greedy(model, lambda rows, steps: _prepare(model, img, rows, steps),
+                   lambda a, *args: L.lo_decoder_greedy_hist(ctypes.byref(a), *args),
+                   start_id, end_id, max_length_formula, return_attention)
+
+
+def _greedy(model, prepare, launch, start_id, end_id, max_length_formula, return_attention):
+    """The greedy loop of any decoder flavour: prepare(rows_per_img, max_steps) -> (args, workspace, N) encodes the images;
+    launch(args, start_id, end_id, max_steps, tokens, finished, fin_hist, stream) runs the C loop."""
     max_steps = max_length_formula + 2
     with torch.no_grad():
-        a, ws, N = _prepare(model, img, 1, max_steps)
+        a, ws, N = prepare(1, max_steps)
         dev = model.device
         tokens = torch.zeros(N, max_steps, dtype=torch.int64, device=dev)
         finished = torch.zeros(N, dtype=torch.int32, device=dev)
         hist = torch.zeros(N, max_steps, dtype=torch.int32, device=dev)
-        check(L.lo_decoder_greedy_hist(ctypes.byref(a), int(start_id), int(end_id), max_steps, tokens.data_ptr(), finished.data_ptr(),
-                                       hist.data_ptr(), stream_ptr()))
+        check(launch(a, int(start_id), int(end_id), max_steps, tokens.data_ptr(), finished.data_ptr(), hist.data_ptr(), stream_ptr()))
         n = _n_steps(hist.cpu())
         if return_attention:
             return tokens[:, :n].cpu(), ws["t"]["alphas"][:, :n].float().cpu()
@@ -77,12 +89,19 @@ def beam_decode(model, img, start_id, end_id, beam_size=5, max_length_formula=15
     (img2seq.py:210).  ``div_gamma`` / ``div_prob``: the diversity penalty of beam_search_decoder_cell.py:258-287 (off when
     gamma == 1 or prob == 0, as in configs/model.json:15-16); its Bernoulli draws come from the in-kernel Philox stream seeded
     by ``div_seed`` (default: torch's initial seed), or from ``div_u`` — uniforms [steps, N*beam, V] — when given (tests)."""
+    L = _lib.lib()
+    return _beam(model, lambda rows, steps: _prepare(model, img, rows, steps),
+                 lambda a, *args: L.lo_decoder_beam_div(ctypes.byref(a), *args),
+                 start_id, end_id, beam_size, max_length_formula, finalize, div_gamma, div_prob, div_u, div_seed)
+
+
+def _beam(model, prepare, launch, start_id, end_id, beam_size, max_length_formula, finalize, div_gamma, div_prob, div_u, div_seed):
+    """The beam loop of any decoder flavour (see _greedy); launch takes the arguments of lo_decoder_beam_div after the args block."""
     if finalize not in ("reference", "backtrack"):
         raise NotImplementedError("finalize must be 'reference' or 'backtrack'")
-    L = _lib.lib()
     max_steps = max_length_formula + 2
     with torch.no_grad():
-        a, ws, N = _prepare(model, img, beam_size, max_steps)
+        a, ws, N = prepare(beam_size, max_steps)
         dev = model.device
         ids = torch.zeros(N, max_steps, beam_size, dtype=torch.int64, device=dev)
         parents = torch.zeros_like(ids)
@@ -97,10 +116,9 @@ def beam_decode(model, img, start_id, end_id, beam_size=5, max_length_formula=15
         elif div_on:
             seed = torch.initial_seed() if div_seed is None else int(div_seed)
             state = torch.tensor([seed & 0x7FFFFFFFFFFFFFFF, 0], dtype=torch.int64, device=dev)
-        check(L.lo_decoder_beam_div(ctypes.byref(a), int(start_id), int(end_id), max_steps, ids.data_ptr(), parents.data_ptr(),
-                                    hist.data_ptr(), logp.data_ptr(), float(div_gamma), float(div_prob),
-                                    u_dev.data_ptr() if u_dev is not None else None,
-                                    state.data_ptr() if state is not None else None, stream_ptr()))
+        check(launch(a, int(start_id), int(end_id), max_steps, ids.data_ptr(), parents.data_ptr(), hist.data_ptr(), logp.data_ptr(),
+                     float(div_gamma), float(div_prob), u_dev.data_ptr() if u_dev is not None else None,
+                     state.data_ptr() if state is not None else None, stream_ptr()))
         n = _n_steps(hist.cpu())
         ids, parents = ids[:, :n].cpu(), parents[:, :n].cpu()
         if finalize == "backtrack":

@@ -316,9 +316,10 @@ class DecoderWithAttention(nn.Module):
                                 1, 0, 0, 0, ptr(S.f32(n + ".bias")), 0, 0, _lib.LO_IMPL_SIMT, st))
             return hc[0], hc[1]
 
-    def run_phase(self, ws, phase, backward):
+    def run_phase(self, ws, phase, backward, with_loss=True):
         """Extension hook (a second layer between the cell and fc, latex_ocr_b200/ext.py): re-enter the C entry points with
-        ``lo_decoder_args.phase`` = 1 (time loop only) or 2 (fc head + loss only) on the argument block of run_forward."""
+        ``lo_decoder_args.phase`` = 1 (time loop only) or 2 (fc head + loss only) on the argument block of run_forward.
+        ``with_loss=False``: forward of the head without the loss (the workspace of a no-gradient run_forward)."""
         a = ws["args"]
         a.phase = int(phase)
         try:
@@ -326,7 +327,7 @@ class DecoderWithAttention(nn.Module):
             if backward:
                 check(L.lo_decoder_backward(ctypes.byref(a), stream_ptr()))
             else:
-                check(L.lo_decoder_forward(ctypes.byref(a), 1, stream_ptr()))
+                check(L.lo_decoder_forward(ctypes.byref(a), 1 if with_loss else 0, stream_ptr()))
         finally:
             a.phase = 0
 

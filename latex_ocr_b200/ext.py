@@ -13,6 +13,10 @@ is no reference code to restate; semantics are defined HERE and checked against 
 
 Both LSTMs run on ``lo_lstm_seq_forward/backward`` (csrc/lo_lstmseq.cuh): hoisted input projection, one recurrent GEMM + one cell
 kernel per step, hand-derived backward with hoisted weight gradients.
+
+Decoding (``greedy_decode`` / ``beam_decode``, same loop rules and outputs as latex_ocr_b200.decode) runs layer 2 inside the time
+loop, step by step, because token t+1 depends on fc(h2_t): ``lo_decoder2_greedy_hist`` / ``lo_decoder2_beam_div``
+(csrc/lo_decoder2.cuh).  In beam search layer 2's state follows the parents like layer 1's.
 """
 import ctypes
 import math
@@ -20,7 +24,7 @@ import math
 import torch
 import torch.nn as nn
 
-from . import _lib
+from . import _lib, decode
 from ._lib import check, ptr, stream_ptr
 from .img2seq import Img2SeqModel
 from .params import FlatStore, LRUCache, ParamHolder
@@ -33,10 +37,13 @@ def _make_struct():
     class LstmSeqArgs(ctypes.Structure):
         _fields_ = _lib._parse_struct(text, "lo_lstm_seq_args")
 
-    return LstmSeqArgs
+    class Dec2Args(ctypes.Structure):
+        _fields_ = _lib._parse_struct(text, "lo_dec2_args")
+
+    return LstmSeqArgs, Dec2Args
 
 
-LstmSeqArgs = _make_struct()
+LstmSeqArgs, Dec2Args = _make_struct()
 _bound = False
 
 
@@ -55,6 +62,16 @@ def _bind():
         fn = getattr(L, name)
         fn.argtypes = [P, ctypes.c_void_p]
         fn.restype = ctypes.c_int
+    L.lo_sizeof_dec2_args.restype = ctypes.c_int64
+    if L.lo_sizeof_dec2_args() != ctypes.sizeof(Dec2Args):
+        raise _lib.LatexOcrB200Error("lo_dec2_args layout mismatch — rebuild")
+    L.lo_dec2_workspace_bytes.restype = ctypes.c_int64
+    L.lo_dec2_workspace_bytes.argtypes = [ctypes.c_int, ctypes.c_int]
+    PD, P2 = ctypes.POINTER(_lib.DecoderArgs), ctypes.POINTER(Dec2Args)
+    vp, i32, i64, f32 = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_float
+    L.lo_decoder2_greedy_hist.argtypes = [PD, P2, i64, i64, i32, vp, vp, vp, vp]
+    L.lo_decoder2_beam_div.argtypes = [PD, P2, i64, i64, i32, vp, vp, vp, vp, f32, f32, vp, vp, vp]
+    L.lo_decoder2_greedy_hist.restype = L.lo_decoder2_beam_div.restype = ctypes.c_int
     _bound = True
     return L
 
@@ -197,6 +214,7 @@ class DecoderLayer2(nn.Module):
                 p_.uniform_(-b, b)
         self._shadow_fresh = False
         self._x = LRUCache()
+        self._dec = LRUCache()
 
     def _load_from_state_dict(self, *a, **k):
         super()._load_from_state_dict(*a, **k)
@@ -221,6 +239,22 @@ class DecoderLayer2(nn.Module):
         a.hs_row, a.hs_step = T * D, D
         check(_bind().lo_lstm_seq_forward(ctypes.byref(a), stream_ptr()))
 
+    def decode_args(self, B):
+        """lo_dec2_args of the decode loops for B rows (layer 2 inside the time loop; workspace cached per B)."""
+        self.sync_shadow()
+        ent = self._dec.get(B)
+        S = self.store
+        if ent is None:
+            nbytes = int(_bind().lo_dec2_workspace_bytes(B, self.D))
+            ent = self._dec[B] = {"a": Dec2Args(), "ws": torch.empty(nbytes, dtype=torch.uint8, device=S.device)}
+        a = ent["a"]
+        a.D, a.dt = self.D, _dt(self.precision)
+        a.impl = _lib.LO_IMPL_TC if (self.impl == "tc" and self.precision == "bf16") else _lib.LO_IMPL_SIMT
+        a.w_ih, a.w_hh = S.w("cell.weight_ih").data_ptr(), S.w("cell.weight_hh").data_ptr()
+        a.b_ih, a.b_hh = S.f32("cell.bias_ih").data_ptr(), S.f32("cell.bias_hh").data_ptr()
+        a.ws = ent["ws"].data_ptr()
+        return a
+
     def backward_inplace(self, dhd):
         """dhd: fp32 [B,T,D] holding d loss / d h2 — replaced IN PLACE by d loss / d dropout(h1)."""
         B, T, D = dhd.shape
@@ -232,9 +266,40 @@ class DecoderLayer2(nn.Module):
         check(_bind().lo_lstm_seq_backward(ctypes.byref(a), stream_ptr()))
 
 
+def _encode(model, img):
+    """CNN -> row biLSTM: the storage-dtype encoder output [N,H',W',512] the two-layer decoder attends over."""
+    feat = model.encoder.forward_raw(img.to(model.device).float(), need_grad=False)
+    return model.row_encoder.forward_raw(feat)
+
+
+def _prepare(model, img):
+    return lambda rows, steps: decode._prepare_enc(model, _encode(model, img), rows, steps)
+
+
+def greedy_decode(model, img, start_id, end_id, max_length_formula=150, return_attention=False):
+    """decode.greedy_decode for an Img2SeqRowModel: token ids [N, steps] (CPU int64), with ``return_attention=True`` also the
+    attention weights [N, steps, R]."""
+    L = _bind()
+    return decode._greedy(model, _prepare(model, img),
+                          lambda a, *args: L.lo_decoder2_greedy_hist(ctypes.byref(a), ctypes.byref(model.layer2.decode_args(a.B)), *args),
+                          start_id, end_id, max_length_formula, return_attention)
+
+
+def beam_decode(model, img, start_id, end_id, beam_size=5, max_length_formula=150, finalize="reference", div_gamma=1, div_prob=0,
+                div_u=None, div_seed=None):
+    """decode.beam_decode for an Img2SeqRowModel: (ids [N, beam, steps], log_probs [N, beam]) on the CPU; same finalize modes and
+    diversity penalty."""
+    L = _bind()
+    return decode._beam(model, _prepare(model, img),
+                        lambda a, *args: L.lo_decoder2_beam_div(ctypes.byref(a), ctypes.byref(model.layer2.decode_args(a.B)), *args),
+                        start_id, end_id, beam_size, max_length_formula, finalize, div_gamma, div_prob, div_u, div_seed)
+
+
 class Img2SeqRowModel(Img2SeqModel):
     """EncoderCNN -> RowEncoder -> attention decoder with a second LSTM layer (extension).  Same trainer surface as
-    Img2SeqModel (getLoss / train_step / train / ...); decoding (predict_batch) is not offered for this variant."""
+    Img2SeqModel (getLoss / train_step / train / evaluate / write_prediction); evaluation decodes and scores this model
+    (``ext.greedy_decode`` / ``ext.beam_decode``).  ``predict_batch`` is not offered yet: call ``ext.greedy_decode`` /
+    ``ext.beam_decode`` directly."""
 
     def getModel(self, model_name="Img2Seq"):
         super().getModel(model_name)
@@ -253,7 +318,30 @@ class Img2SeqRowModel(Img2SeqModel):
         self.layer2.store.set_lr(lr)
 
     def predict_batch(self, *a, **k):
-        raise NotImplementedError("the row-encoder / two-layer extension offers the training path only")
+        raise NotImplementedError("predict_batch is not offered for the row-encoder / two-layer extension: "
+                                  "use latex_ocr_b200.ext.greedy_decode / ext.beam_decode")
+
+    def _decode_ids(self, images, start_id=None, decoding=None, beam_size=None):
+        return self._decode_ids_with(greedy_decode, beam_decode, images, start_id, decoding, beam_size)
+
+    def _teacher_forced_ce(self, img, formula_t, lens, start_id):
+        """Img2SeqModel._teacher_forced_ce on the two-layer model, run as _step_body runs it but without gradient or dropout:
+        phase 1 (time loop of layer 1, writes hd = h1) -> layer 2 over the sequence -> phase 2 (fc head)."""
+        inp = torch.cat([torch.full((formula_t.shape[0], 1), start_id, dtype=torch.int64), formula_t], dim=1)
+        with torch.no_grad():
+            enc = _encode(self, img)
+            N, C = enc.shape[0], enc.shape[3]
+            lens_s, sort_ind = (lens + 1).squeeze(1).sort(dim=0, descending=True)       # seq2seq_torch.py:286
+            si = sort_ind.to(self.device)
+            enc_s = enc.view(N, -1, C)[si].contiguous()
+            caps = inp.to(self.device)[si].contiguous()
+            dl = (lens_s - 1).tolist()
+            dec = self.decoder
+            ws = dec.run_forward(enc_s, caps, dl, with_loss=False, need_grad=False, phase=1)
+            self.layer2.forward_inplace(ws["t"]["hd"])
+            dec.run_phase(ws, 2, backward=False, with_loss=False)
+            preds = ws["t"]["logits"][:, :, :dec.vocab_size]
+            return self._ce_sum(preds, caps[:, 1:], dl)
 
     def _keepalive(self):
         keep = super()._keepalive()

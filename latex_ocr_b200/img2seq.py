@@ -267,19 +267,23 @@ class Img2SeqModel:
         """Token ids per hypothesis rank: list[n_hyp][N] of id lists (NOT truncated), as ``pred_test.ids`` after the
         reshapes of img2seq.py:236-241 / :265-268."""
         from . import decode
+        return self._decode_ids_with(decode.greedy_decode, decode.beam_decode, images, start_id, decoding, beam_size)
+
+    def _decode_ids_with(self, greedy_decode, beam_decode, images, start_id, decoding, beam_size):
+        """_decode_ids on the given greedy / beam decode functions (signatures of latex_ocr_b200.decode's)."""
         decoding = decoding or getattr(self._config, "decoding", "greedy")
         end_id = self._vocab.id_end if self._vocab is not None else self._n_tok - 1
         start_id = end_id - 1 if start_id is None else start_id          # default: the PAD id (no START in the torch flavour)
         L = int(getattr(self._config, "max_length_formula", 150))
         self.train_mode(False)
         if decoding == "greedy":
-            return [decode.greedy_decode(self, images, start_id, end_id, L).tolist()], end_id
+            return [greedy_decode(self, images, start_id, end_id, L).tolist()], end_id
         if decoding != "beam_search" and decoding != "beam":
             raise NotImplementedError("decoding=%r: 'greedy' or 'beam_search' (model.json:13)" % (decoding,))
         beam = int(beam_size or getattr(self._config, "beam_size", 5))
-        ids, _ = decode.beam_decode(self, images, start_id, end_id, beam, L,
-                                    div_gamma=float(getattr(self._config, "div_gamma", 1)),
-                                    div_prob=float(getattr(self._config, "div_prob", 0)))
+        ids, _ = beam_decode(self, images, start_id, end_id, beam, L,
+                             div_gamma=float(getattr(self._config, "div_gamma", 1)),
+                             div_prob=float(getattr(self._config, "div_prob", 0)))
         return [ids[:, k].tolist() for k in range(beam)], end_id
 
     def predict_batch(self, images, start_id=None, decoding=None, beam_size=None):
@@ -308,7 +312,11 @@ class Img2SeqModel:
         inp = torch.cat([torch.full((formula_t.shape[0], 1), start_id, dtype=torch.int64), formula_t], dim=1)
         enc = self.encoder(img.to(self.device))
         preds, caps, dl, _, _ = self.decoder(enc, inp.to(self.device), lens + 1)
-        tgt = caps[:, 1:]
+        return self._ce_sum(preds, caps[:, 1:], dl)
+
+    @staticmethod
+    def _ce_sum(preds, tgt, dl):
+        """(sum of CE, number of tokens) over the first dl[b] steps of each row of the logits preds [B,T,V]."""
         ce_sum, n_tok = 0.0, 0
         for b, n in enumerate(dl):
             lp = torch.log_softmax(preds[b, :n].float(), dim=-1)                 # host-side metric arithmetic (plumbing)
